@@ -4,10 +4,14 @@
 
     python bench.py --gpus N --steps K --warmup W [--workload servos|pendulum|mpc]
     python bench.py --impl reference ...      # CPU arm (oracle port on host cores)
+    python bench.py --gpus 1 ... --dump-outputs DIR
 
 A "step" is one pass of the hot path over one batch: one 5 ms control tick
 (5 x 1 ms physics substeps) of every env of the batch = one kernel launch.
-Prints ONE JSON line on rank 0.
+Prints ONE JSON line on rank 0. The inputs are seeded: with the same arguments
+every run times the same computation, and ``--dump-outputs DIR`` writes the
+outputs of the last timed step as ``DIR/<name>.npy`` so that two builds can be
+compared output for output.
 
 Workloads (BASELINE.json configs):
   servos   (default) configs[2]/[4]: 65536 UpkieServos envs per GPU, pure torque
@@ -45,6 +49,25 @@ B_ALG = {"servos": 542 + 284 + 3 * 4 * 2 + 4 * 4 * 2, "pendulum": 346 + 3 * 4 * 
 B_ALG_SERVOS_COMPACT = B_ALG["servos"] - 48 - 5
 N_ACTION_BUFFERS = 16
 ROLLOUT_T = 32  # steps per rollout gather; shortened to K // 4 when the timed region has fewer than 128 steps
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(directory, arrays):
+    """Write ``{name: tensor}`` (outputs of the last timed step, first axis = env) as ``directory/<name>.npy``, float64
+    kept, everything else as float32. Above DUMP_LIMIT_BYTES in all, every array keeps the same seeded sample of envs,
+    whose indices go to ``env_index.npy``."""
+    host = {name: t.detach().cpu().numpy() for name, t in arrays.items()}
+    host = {name: a.astype(np.float64 if a.dtype == np.float64 else np.float32) for name, a in host.items()}
+    n = next(iter(host.values())).shape[0]
+    total = sum(a.nbytes for a in host.values())
+    if total > DUMP_LIMIT_BYTES:
+        keep = DUMP_LIMIT_BYTES * n // (total + 8 * n)
+        index = np.sort(np.random.default_rng(0).choice(n, keep, replace=False))
+        host = {name: a[index] for name, a in host.items()}
+        host["env_index"] = index.astype(np.float64)
+    os.makedirs(directory, exist_ok=True)
+    for name, a in host.items():
+        np.save(os.path.join(directory, f"{name}.npy"), a)
 
 
 def read_peaks():
@@ -344,11 +367,17 @@ def main():
     ap.add_argument("--envs-per-gpu", type=int, default=None)
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-other-workloads", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the outputs of the last timed step as DIR/<name>.npy (servos, pendulum, mpc; 1 GPU)")
     args = ap.parse_args()
 
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "b200" or args.workload == "plumbing" or world > 1):
+        ap.error("--dump-outputs: the servos, pendulum and mpc workloads of the GPU arm on one GPU")
 
     if args.impl == "reference":
         run_reference_arm(args, rank, world)
@@ -821,6 +850,11 @@ def bench_env(args, torch, dist, dev, rank, world, model, K, W):
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
     t_ms = float(t.item()) / K
     launches = env.sim.launches - launches0
+    if args.dump_outputs:
+        last = Wa + K - 1  # the rollout slot the last timed step wrote; nothing writes it after the timed region
+        outputs = rollouts[(last // T_roll) % 2].slot(last)
+        names = ("obs", "reward", "terminated", "truncated")
+        dump_outputs(args.dump_outputs, {name: out for name, out in zip(names, outputs) if out is not None})
 
     if os.environ.get("UPKIE_BENCH_DEVICE_ONLY") == "1":  # exact-mode companion run: no host-buffer kernels in that library
         config = {"workload": "device-only run", "envs_per_gpu": n, "rollout_record": "full",
@@ -998,6 +1032,8 @@ def bench_mpc(args, torch, dev, rank, world, K, W):
         clk.mark_end()
     total_ms = events[0].elapsed_time(events[K])
     per_step = np.array([events[k].elapsed_time(events[k + 1]) for k in range(K)])
+    if args.dump_outputs:  # before the host-array loop below overwrites it
+        dump_outputs(args.dump_outputs, {"commanded_velocity": mpc.commanded_velocity})
     xh = [x.cpu().numpy() for x in xs[:4]]
     vth, ch = vt.cpu().numpy(), contact.cpu().numpy()
     Ke = max(10, min(K, 400))

@@ -7,7 +7,8 @@ Run in the build container:  python tests/golden/make_ref_spine_golden.py
 ``oracle/_ref/libupkie_ref_spine.so`` is the reference's upkie/cpp/observers/*.cpp and upkie/cpp/controllers/*.cpp
 compiled unmodified and in place (oracle/Makefile ``ref``; Eigen / palimpsest / spdlog replaced by the stand-in
 headers of oracle/standin/), behind the flat-array glue of oracle/ref_spine_shim.cpp. This script drives it with
-seeded inputs and stores inputs + outputs in tests/golden/ref_spine_runs.json, so that the oracle's restatement
+seeded inputs and stores inputs + outputs in tests/golden/ref_spine_runs.json (and whole output rows of the
+side-by-side run in tests/golden/ref_spine_side_by_side.json), so that the oracle's restatement
 (ObserverPipelineOracle, WheelBalancerOracle) stays pinned on machines where the reference tree, and therefore the
 library, are absent.
 """
@@ -19,6 +20,8 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 OUT = os.path.join(os.path.dirname(os.path.abspath(__file__)), "ref_spine_runs.json")
+OUT_SIDE = os.path.join(os.path.dirname(os.path.abspath(__file__)), "ref_spine_side_by_side.json")
+SIDE_BY_SIDE_EVERY = 4
 sys.path.insert(0, ROOT)
 
 
@@ -66,6 +69,20 @@ def main():
     with open(OUT, "w") as f:
         json.dump(out, f)
     print("wrote", OUT, os.path.getsize(OUT) // 1024, "KB")
+
+    # whole observer rows and whole 6 x 6 controller outputs (NaN -> None) of the library on the inputs of
+    # test_ref_spine.py::test_reference_library_side_by_side, every SIDE_BY_SIDE_EVERY-th step to keep the file small
+    freq, stream = 500, 7
+    ref = O.RefSpine(A.default_observer_config(model, float(freq)), A.default_wheel_balancer_config(float(freq)), freq)
+    obs_rows = [ref.observers_step(r).tolist() for r in inputs.observer_inputs(A, stream)]
+    ctrl_rows = [[None if v != v else v for v in ref.controllers_step(obs3, target, act).reshape(36).tolist()]
+                 for obs3, target, act in inputs.controller_inputs(stream)]
+    every = SIDE_BY_SIDE_EVERY
+    side = {"generator": "tests/golden/make_ref_spine_golden.py", "spine_frequency": freq, "stream": stream,
+            "every": every, "observers": obs_rows[::every], "controllers": ctrl_rows[::every]}
+    with open(OUT_SIDE, "w") as f:
+        json.dump(side, f)
+    print("wrote", OUT_SIDE, os.path.getsize(OUT_SIDE) // 1024, "KB")
 
 
 if __name__ == "__main__":

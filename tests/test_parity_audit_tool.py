@@ -1,7 +1,8 @@
 # SPDX-License-Identifier: Apache-2.0
 """tools/parity_audit.py: the record / compare logic, exercised on the reference's own ``PyBulletBackend`` (loaded
-unmodified from the reference tree, ``pybullet`` replaced by the stand-in whose physics is oracle/). Skipped where the
-reference tree is absent. The tool's purpose - a run against a REAL PyBullet - needs a machine that has one."""
+unmodified from the reference tree, ``pybullet`` replaced by the stand-in whose physics is oracle/), and on that
+backend's observations as recorded in tests/golden/reference_suite_runs.json where the tree is absent. The tool's
+purpose - a run against a REAL PyBullet - needs a machine that has one."""
 import importlib.util
 import os
 import sys
@@ -37,9 +38,73 @@ def test_scenarios_are_open_loop_and_seeded(audit):
         audit.scenario_actions("torques", 5, 0.005, 2, tau_max))
 
 
+def _check_recordings(audit, paths, ticks):
+    """Three "torques" recordings: seeds 0, 0 and 1."""
+    header, records = audit.load(paths[0])
+    assert header["scenario"] == "torques" and len(records) == ticks + 1
+    assert records[0]["tick"] == 0 and records[-1]["tick"] == ticks
+    assert set(records[1]["action"]["servo"]) == set(audit.JOINTS)
+    same = audit.compare(paths[0], paths[1])
+    assert "servo.left_knee.position" in same and "imu.orientation" in same
+    assert max(max(row.values()) for row in same.values()) == 0.0  # same inputs, same backend: identical
+    other = audit.compare(paths[0], paths[2])  # different torques: the table shows it
+    assert other["servo.left_knee.velocity"][ticks] > 1e-2
+    assert sorted(other["servo.left_knee.velocity"]) == [1, 2, 5, 10, 20, 40]
+    audit.print_table(other)
+
+
+class _ReplayBackend:
+    """Serves, tick by tick, the observations the reference's PyBulletBackend returned for the same actions
+    (tests/golden/make_reference_suite_golden.py)."""
+
+    def __init__(self, run):
+        self._keys, self._sizes, self._rows = run["keys"], run["sizes"], run["observations"]
+        self._k = 0
+
+    def _observation(self):
+        row, out, i = self._rows[self._k], {}, 0
+        for key, size in zip(self._keys, self._sizes):
+            out[key] = row[i:i + size]
+            i += size
+        self._k += 1
+        return out
+
+    def reset(self, init_state):
+        self._k = 0
+        return self._observation()
+
+    def step(self, action):
+        return self._observation()
+
+
+def _record_and_compare_recorded_runs(audit, tmp_path):
+    import hashlib
+    import json
+
+    with open(os.path.join(os.path.dirname(__file__), "golden", "reference_suite_runs.json")) as f:
+        golden = json.load(f)["parity_audit"]
+    from upkie_b200.robot_state import RobotState
+
+    dt, ticks = golden["dt"], golden["ticks"]
+    paths = []
+    for run, scenario_seed in enumerate((0, 0, 1)):
+        recorded = golden["runs"][str(scenario_seed)]
+        actions = audit.scenario_actions("torques", ticks, dt, scenario_seed, recorded["tau_max"])
+        assert hashlib.sha256(repr(actions).encode()).hexdigest() == recorded["actions_sha256"]  # what the reference saw
+        header = {"format": "upkie_b200.parity_audit/1", "backend": "pybullet", "scenario": "torques",
+                  "seed": 0, "dt": dt, "ticks": ticks, "urdf": "robot.urdf"}
+        path = str(tmp_path / f"recorded{run}.mpack")
+        audit.record(_ReplayBackend(recorded), RobotState, actions, header, path)
+        paths.append(path)
+    _check_recordings(audit, paths, ticks)
+
+
 def test_record_and_compare_on_the_reference_backend(audit, tmp_path):
+    """On the reference backend's recorded observations everywhere, and on the backend itself where the reference
+    tree is present."""
+    _record_and_compare_recorded_runs(audit, tmp_path)
     if not os.path.exists(os.path.join(REF, "upkie", "envs", "backends", "pybullet_backend.py")):
-        pytest.skip("reference tree not present on this machine")
+        return
     sys.path.insert(0, os.path.join(os.path.dirname(__file__), "golden"))
     import make_backend_golden as bg
     import make_wrapper_golden as wg
@@ -84,17 +149,7 @@ def test_record_and_compare_on_the_reference_backend(audit, tmp_path):
             audit.record(backend, robot_state_cls, actions, header, path)
             backend.close()
             paths.append(path)
-        header, records = audit.load(paths[0])
-        assert header["scenario"] == "torques" and len(records) == ticks + 1
-        assert records[0]["tick"] == 0 and records[-1]["tick"] == ticks
-        assert set(records[1]["action"]["servo"]) == set(audit.JOINTS)
-        same = audit.compare(paths[0], paths[1])
-        assert "servo.left_knee.position" in same and "imu.orientation" in same
-        assert max(max(row.values()) for row in same.values()) == 0.0  # same inputs, same backend: identical
-        other = audit.compare(paths[0], paths[2])  # different torques: the table shows it
-        assert other["servo.left_knee.velocity"][ticks] > 1e-2
-        assert sorted(other["servo.left_knee.velocity"]) == [1, 2, 5, 10, 20, 40]
-        audit.print_table(other)
+        _check_recordings(audit, paths, ticks)
     finally:
         for k in [k for k in sys.modules if k.split(".")[0] in names]:
             del sys.modules[k]

@@ -108,20 +108,29 @@ def test_kernel_arithmetic_matches_the_reference_cpp(golden, model, stream):
 
 
 def test_reference_library_side_by_side(model, oracle_lib):
-    """Direct comparison with the compiled reference where oracle/_ref/ exists (fresh inputs, not the golden ones)."""
+    """Whole observer rows and whole controller outputs versus the compiled reference (inputs other than the golden
+    ones above): its outputs stored in tests/golden/ref_spine_side_by_side.json (every `every`-th step), and the
+    library itself, step by step, where oracle/_ref/ exists."""
     O = oracle_lib
-    if not os.path.exists(O.REF_SPINE_PATH):
-        pytest.skip("oracle/_ref/libupkie_ref_spine.so not built (reference tree absent)")
-    freq = 500
+    side = json.load(open(os.path.join(os.path.dirname(__file__), "golden", "ref_spine_side_by_side.json")))
+    freq, stream, every = side["spine_frequency"], side["stream"], side["every"]
     ocfg = A.default_observer_config(model, float(freq))
     wcfg = A.default_wheel_balancer_config(float(freq))
-    ref = O.RefSpine(ocfg, wcfg, freq)
+    ref = O.RefSpine(ocfg, wcfg, freq) if os.path.exists(O.REF_SPINE_PATH) else None
     oo = OracleObservers(oracle_lib, ocfg, 1)
     ob = OracleBalancer(oracle_lib, wcfg, 1)
-    rows = inputs.observer_inputs(A, 7)
+    rows = inputs.observer_inputs(A, stream)
     for k in range(inputs.N_STEPS):
-        assert np.allclose(oo.step(rows[k:k + 1])[0], ref.observers_step(rows[k]), rtol=1e-12, atol=1e-12), k
-    for k, (obs3, target, act) in enumerate(inputs.controller_inputs(7)):
+        mine = oo.step(rows[k:k + 1])[0]
+        if k % every == 0:
+            assert np.allclose(mine, side["observers"][k // every], rtol=1e-12, atol=1e-12), k
+        if ref is not None:
+            assert np.allclose(mine, ref.observers_step(rows[k]), rtol=1e-12, atol=1e-12), k
+    for k, (obs3, target, act) in enumerate(inputs.controller_inputs(stream)):
         mine, _ = ob.step(obs3.reshape(1, 3), None if target is None else target.reshape(1, 2), act.reshape(1, 6, 6))
-        theirs = ref.controllers_step(obs3, target, act)
-        assert np.allclose(mine.reshape(6, 6), theirs, rtol=1e-12, atol=1e-12, equal_nan=True), k
+        if k % every == 0:
+            stored = np.array([np.nan if v is None else v for v in side["controllers"][k // every]]).reshape(6, 6)
+            assert np.allclose(mine.reshape(6, 6), stored, rtol=1e-12, atol=1e-12, equal_nan=True), k
+        if ref is not None:
+            theirs = ref.controllers_step(obs3, target, act)
+            assert np.allclose(mine.reshape(6, 6), theirs, rtol=1e-12, atol=1e-12, equal_nan=True), k

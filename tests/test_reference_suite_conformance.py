@@ -1,17 +1,23 @@
 # SPDX-License-Identifier: Apache-2.0
 """Runs the REFERENCE'S OWN unit tests against this package's mirrors of the reference's host-side types.
 
-Where the reference tree is present (the build container), its test files for the types we mirror are loaded as they
-are and executed with ``upkie.utils.robot_state`` / ``robot_state_randomization`` / ``external_force`` aliased to
-``upkie_b200``'s classes: a user switching packages keeps the behaviour those tests specify. Skipped elsewhere (the
-GPU box and fresh clones have no /root/reference; nothing else in the suite depends on it)."""
+Where the reference tree is present, its test files for the types we mirror are loaded as they are and executed with
+``upkie.utils.robot_state`` / ``robot_state_randomization`` / ``external_force`` aliased to ``upkie_b200``'s classes:
+a user switching packages keeps the behaviour those tests specify. Everywhere, the same comparisons run against what
+the reference's code produced when tests/golden/make_reference_suite_golden.py ran it (reference_suite_runs.json)."""
+import hashlib
 import importlib.util
+import json
 import os
 import sys
 import types
 import unittest
 
+import numpy as np
 import pytest
+
+sys.path.insert(0, os.path.join(os.path.dirname(__file__), "golden"))
+import reference_suite_probes as probes  # noqa: E402
 
 REF_TESTS = os.path.join(os.environ.get("UPKIE_REFERENCE", "/root/reference"), "tests")
 
@@ -21,6 +27,12 @@ CASES = [
     ("utils/test_rotations.py", "rotation_matrix_from_rpy of the URDF loader"),
     ("utils/test_point_contact.py", "PointContact of Backend.get_contact_points"),
 ]
+
+
+@pytest.fixture(scope="module")
+def golden():
+    with open(os.path.join(os.path.dirname(__file__), "golden", "reference_suite_runs.json")) as f:
+        return json.load(f)
 
 
 @pytest.fixture()
@@ -59,10 +71,14 @@ def aliased_upkie():
 
 
 @pytest.mark.parametrize("rel,what", CASES)
-def test_reference_unit_tests_pass_on_our_mirrors(aliased_upkie, rel, what):
+def test_reference_unit_tests_pass_on_our_mirrors(aliased_upkie, golden, rel, what):
+    """The probes of tests/golden/reference_suite_probes.py (the inputs of the reference's test file and a few seeded
+    ones) give on our mirrors what they gave on the reference's classes; the test file itself where it is present."""
+    problems = probes.mismatches(probes.PROBES[rel](sys.modules), golden["unit_probes"][rel])
+    assert not problems, f"{what}: {problems[:5]}"
     path = os.path.join(REF_TESTS, rel)
     if not os.path.exists(path):
-        pytest.skip("reference tree not present on this machine")
+        return
     spec = importlib.util.spec_from_file_location("reference_test_" + os.path.basename(rel)[:-3], path)
     mod = importlib.util.module_from_spec(spec)
     spec.loader.exec_module(mod)
@@ -74,18 +90,63 @@ def test_reference_unit_tests_pass_on_our_mirrors(aliased_upkie, rel, what):
     assert not problems, f"{what}: {problems}"
 
 
+def _replay_backend_suite(golden, joint_limits, tmp_path, oracle_lib):
+    """The runs behind the reference's backend suite, recorded from its PyBulletBackend on the stand-in whose physics
+    is oracle/, replayed by the oracle's restatement of that backend: every step's pitch and the whole spine
+    observation at the recorded checkpoints."""
+    from test_backend_golden import _action, _compare, _row64
+    from upkie_b200 import _abi as A
+    from upkie_b200.model import Model
+    from upkie_b200.urdf import write_urdf
+
+    g = golden["backend_suite"][str(joint_limits)]
+    assert g["suite"]["tests"] >= 4
+    assert not [p for p in g["suite"]["problems"] if not (joint_limits and "test_fall_pitch" in p)], g["suite"]
+    urdf = str(tmp_path / "robot.urdf")
+    write_urdf(Model.standard_upkie(), urdf, split_fixed_links=False)
+    model = Model.from_urdf(urdf)
+    upright = np.zeros(A.INIT_DIM)
+    upright[2], upright[3] = 0.6, 1.0  # RobotState(position_base_in_world=[0, 0, 0.6]) of the suite's setUp
+    action, absent = _action([None] * 6)  # step(action={}): no joint commanded
+    for scenario, run in g["runs"].items():
+        cfg = A.default_sim_config()
+        cfg.joint_limits = joint_limits
+        osim = oracle_lib.OracleSim(model, cfg, 1, threads=1)
+        osim.reset(upright.reshape(1, -1))
+        if scenario == "yawed":  # backend._reset_robot_state(yaw = pi / 2) after setUp's reset
+            osim.set_state(np.asarray(run["state_after_reset_robot_state"]).reshape(1, -1))
+        for t in range(len(run["pitch"]) + 1):
+            if t > 0:
+                osim.step_servos(action.reshape(1, 6, 6))
+                assert abs(osim.spine_obs()[0][A.SP_PITCH] - run["pitch"][t - 1]) < 1e-9, (scenario, t)
+            if str(t) not in run["observations"]:
+                continue
+            mine, ref = osim.spine_obs()[0], _row64(run["observations"][str(t)])
+            if scenario == "yawed" and t == 1:
+                # the backend's IMU finite difference spans its _reset_robot_state, which set_state does not carry
+                for block in (A.SP_IMU_LINACC, A.SP_IMU_RAWACC):
+                    mine[block:block + 3] = ref[block:block + 3]
+            _compare(mine, ref, 1e-8, skip_torque=absent)
+        assert abs(run["pitch"][0]) < 1e-7  # the suite's pitch right after the reset
+        if not joint_limits:
+            assert abs(run["pitch"][-1]) > 0.5  # and the fall within 100 steps
+
+
 @pytest.mark.parametrize("joint_limits", [0, 3])
-def test_reference_pybullet_backend_suite_passes_on_our_physics(tmp_path, joint_limits):
+def test_reference_pybullet_backend_suite_passes_on_our_physics(tmp_path, golden, oracle_lib, joint_limits):
     """tests/envs/backends/test_pybullet_backend.py of the reference (its tests of the REAL PyBullet backend: step
     returns a dict, pitch 0 after a step, the robot falls within 100 un-actuated steps, also from a yawed start)
     executed unmodified with ``pybullet`` replaced by the stand-in whose physics is oracle/ and ``upkie_description``
     pointing at a URDF written by upkie_b200: what the reference expects of Bullet at that level holds for the
     restated physics. With the joint-limit rows on (the default since round 2) the two "fallen at step 100" samples
     depend on the stand-in inertias (tests/test_oracle_pins.py::test_pitch_zero_after_one_step_and_fall_without_action);
-    they are the only tests allowed to deviate, and the oracle pins assert the fall itself."""
+    they are the only tests allowed to deviate, and the oracle pins assert the fall itself. The suite's runs as
+    recorded from the reference (tests/golden/reference_suite_runs.json) are replayed everywhere; the suite itself
+    runs where the reference tree is present."""
+    _replay_backend_suite(golden, joint_limits, tmp_path, oracle_lib)
     path = os.path.join(REF_TESTS, "envs", "backends", "test_pybullet_backend.py")
     if not os.path.exists(path):
-        pytest.skip("reference tree not present on this machine")
+        return
     sys.path.insert(0, os.path.join(os.path.dirname(__file__), "golden"))
     import make_backend_golden as bg
     import make_wrapper_golden as wg
@@ -131,16 +192,40 @@ def test_reference_pybullet_backend_suite_passes_on_our_physics(tmp_path, joint_
         sys.modules.update(saved)
 
 
-def test_reference_model_suite_passes_on_urdfs_written_by_upkie_b200(tmp_path):
+def test_reference_model_suite_passes_on_urdfs_written_by_upkie_b200(tmp_path, golden):
     """tests/model/test_model.py, test_kinematic_tree.py and test_se3.py of the reference, unmodified, run with the
     reference's OWN ``upkie.model`` package while ``upkie_description.URDF_PATH`` / ``cookie_description.URDF_PATH``
     point at URDFs written by ``upkie_b200.urdf.write_urdf`` (left- and right-wheeled stand-ins): wheel radius 0.05,
     wheel base 0.3048, base -> IMU rotation, torso at (0, 0, -0.1), frame names, tire cylinders, left / right
-    wheeledness - every constant the reference pins on its model comes out of our file through its parser."""
-    if not os.path.exists(os.path.join(REF_TESTS, "model", "test_model.py")):
-        pytest.skip("reference tree not present on this machine")
+    wheeledness - every constant the reference pins on its model comes out of our file through its parser.
+    Everywhere: the files written now are byte for byte those on which the suite passed when
+    tests/golden/make_reference_suite_golden.py ran it, and our loader reads out of them what the reference's parser
+    read; the suite itself runs where the reference tree is present."""
     from upkie_b200.model import Model
     from upkie_b200.urdf import write_urdf
+
+    upkie_urdf, cookie_urdf = str(tmp_path / "upkie.urdf"), str(tmp_path / "cookie.urdf")
+    write_urdf(Model.standard_upkie(), upkie_urdf, split_fixed_links=True)
+    right = Model.standard_upkie()
+    right.joint_axis = right.joint_axis.copy()
+    right.joint_axis[[2, 5]] *= -1.0  # wheel axes reversed: a right-wheeled (Cookie-style) robot
+    write_urdf(right, cookie_urdf, split_fixed_links=True)
+    g = golden["model_suite"]
+    assert g["suite"]["tests"] >= 30 and not g["suite"]["problems"], g["suite"]
+    for name, path in (("upkie", upkie_urdf), ("cookie", cookie_urdf)):
+        ref = g["urdfs"][name]
+        with open(path, "rb") as f:
+            assert hashlib.sha256(f.read()).hexdigest() == ref["sha256"], name
+        m = Model.from_urdf(path)
+        assert m.wheel_radius == pytest.approx(ref["wheel_radius"], abs=1e-12)
+        assert m.wheel_base == pytest.approx(ref["wheel_base"], abs=1e-12)
+        assert m.left_wheeled == ref["left_wheeled"]
+        assert np.allclose(m.rotation_base_to_imu, np.asarray(ref["rotation_base_to_imu"]), atol=1e-12)
+        assert [j.name for j in m.joints] == ref["joint_names"]
+        assert [j.name for j in m.upper_leg_joints] == ref["upper_leg_joints"]
+        assert [j.name for j in m.wheel_joints] == ref["wheel_joints"]
+    if not os.path.exists(os.path.join(REF_TESTS, "model", "test_model.py")):
+        return
 
     ref_root = os.path.dirname(REF_TESTS)
     saved = {k: v for k, v in sys.modules.items()
@@ -148,12 +233,6 @@ def test_reference_model_suite_passes_on_urdfs_written_by_upkie_b200(tmp_path):
     for k in saved:
         del sys.modules[k]
     try:
-        upkie_urdf, cookie_urdf = str(tmp_path / "upkie.urdf"), str(tmp_path / "cookie.urdf")
-        write_urdf(Model.standard_upkie(), upkie_urdf, split_fixed_links=True)
-        right = Model.standard_upkie()
-        right.joint_axis = right.joint_axis.copy()
-        right.joint_axis[[2, 5]] *= -1.0  # wheel axes reversed: a right-wheeled (Cookie-style) robot
-        write_urdf(right, cookie_urdf, split_fixed_links=True)
         for name, path in (("upkie_description", upkie_urdf), ("cookie_description", cookie_urdf)):
             stub = types.ModuleType(name)
             stub.URDF_PATH = path
